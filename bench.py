@@ -3,6 +3,7 @@
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--config NAME] [--dtype bf16|fp32]     our arm (sm_100a kernels)
   python bench.py --impl reference [...]                     the reference's CPU algorithm (oracle port) on host cores
+  python bench.py --dump-outputs DIR [...]                   also write what the last timed step computed to DIR/*.npy
 
 Default workload = BASELINE.json configs[1]: SVQA shapes, N=20 clips x 16 frames x 2048-d appearance + 2048-d motion, GloVe-300
 question of L=20 tokens, unit_layers=3, batch 256 per GPU, bf16 activations, full train step (forward, CE + common + HSIC
@@ -21,6 +22,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the tree may be read-only: the bench writes nothing into it
 
 F_, DV = 16, 2048
 CONFIGS = {
@@ -191,6 +193,33 @@ def classify_kernels(prof):
     return counts
 
 
+DUMP_MAX_ELEMS = 1 << 22       # per array: 16 MB in float32, so the four arrays of --dump-outputs stay under 64 MB
+
+
+def dump_outputs(out_dir, model, loss, logits):
+    """--dump-outputs: what the last timed step handed its caller, as float32 DIR/<name>.npy: the loss, the logits, and
+    the updated parameters and their gradients (every trainable parameter flattened, in the model's parameter order, so
+    the files do not depend on the engine's buffer layout). An array above DUMP_MAX_ELEMS elements is replaced by its
+    flattened elements at a fixed seeded sample of positions (the same positions for arrays of the same size)."""
+    import numpy as np
+    import torch
+
+    def sample(t):
+        t = t.detach()
+        if t.numel() <= DUMP_MAX_ELEMS:
+            return t
+        idx = np.sort(np.random.default_rng(0).choice(t.numel(), DUMP_MAX_ELEMS, replace=False))
+        return t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+
+    params = [p for p in model.parameters() if p.requires_grad]
+    arrays = {"loss": loss.reshape(1), "logits": logits,
+              "params": torch.cat([p.detach().reshape(-1) for p in params]),
+              "grads": torch.cat([p.grad.reshape(-1) for p in params])}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), sample(t).float().cpu().numpy())
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -248,6 +277,11 @@ def run_ours(args):
     res = {k: v.to(dev) for k, v in host.items()}
     h2d_bytes = sum(v.numel() * v.element_size() for v in host.values())
 
+    # the warm-up (and capture) steps are real optimizer steps whose reductions are not bit-reproducible: the timed steps
+    # start again from this seeded state, so that every run hands them the same weights and optimizer state
+    state = [eng.flat, eng.m, eng.v, eng.step_dev, eng.seed_dev] + list(model.buffers())
+    initial = [t.clone() for t in state]
+
     use_graph = not args.no_graph
     if use_graph:
         eng.capture(res["app"], res["mot"], res["q"], res["qlen"], res["ans"], warmup=max(3, args.warmup))
@@ -280,6 +314,13 @@ def run_ours(args):
     for _ in range(max(3, args.warmup)):
         step_resident()
     barrier()
+    with torch.no_grad():
+        for t, t0 in zip(state, initial):
+            t.copy_(t0)
+    eng.sync_shadow()
+    eng.step_count = 0
+    del state, initial
+    barrier()
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
@@ -292,6 +333,8 @@ def run_ours(args):
     value = Bl * world * args.steps / (ms_max / 1e3)
     final_loss = float(loss)
     timeouts = eng.dependency_poll_timeouts()           # max over ranks; a non-zero value also poisons the loss with NaN
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, model, loss, eng.last_logits)
 
     # ---- who launched what: one profiled replay, kernels classified by owner (ours / NCCL / ATen)
     kernels = None
@@ -512,7 +555,13 @@ def main():
     ap.add_argument("--no-kernel-census", action="store_true", help="skip the profiled replay that counts kernels by owner")
     ap.add_argument("--no-comm-ab", action="store_true", help="N>1: skip the second capture that measures the exposed all-reduce")
     ap.add_argument("--no-dp-parity", action="store_true", help="N>1: skip the sharded-vs-single-rank gradient check")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's loss, logits, parameters and "
+                    "gradients to DIR/*.npy (float32; seeded samples of the large ones) to compare two builds")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to the CUDA arm (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -6,7 +6,8 @@ container; the fixtures it writes are what pins the oracle (and, through it, the
 
 Stored per config: the reference's outputs in float64 ("truth") and float32 (to record the reference's own
 fp32-vs-fp64 floor), loss terms, and per-parameter gradient summaries (L2 norm + projection on a seeded probe vector)
-for the CE-only loss and for the full training loss of train.py:146-154."""
+for the CE-only loss and for the full training loss of train.py:146-154. A config with embed_samples keeps the aq/mq
+embeddings of that many seeded batch rows only ("embed_rows" holds their indices)."""
 import os
 import sys
 
@@ -24,8 +25,13 @@ CONFIGS = {
     "g2_B3_N20_U3": dict(B=3, N=20, L=9, A=32, V=50, U=3, full=False),
     "g3_B5_N16_U1": dict(B=5, N=16, L=5, A=17, V=40, U=1, full=False),
     # a realistic batch for the train-mode BatchNorm (the three above have 3-5 samples): holds the un-relaxed 2e-2 gradient gate
-    "g4_B16_N20_U3": dict(B=16, N=20, L=12, A=32, V=60, U=3, full=False),
+    "g4_B16_N20_U3": dict(B=16, N=20, L=12, A=32, V=60, U=3, full=False, embed_samples=6),
 }
+
+
+def embed_rows(B, k):
+    """The batch rows whose aq/mq embeddings a fixture keeps when its config sets embed_samples (keeps the file < 1 MB)."""
+    return np.sort(np.random.default_rng(0).choice(B, k, replace=False))
 
 
 def no_dropout(model):
@@ -116,6 +122,10 @@ def main():
             if dt_name == "f64":
                 blob["grad_names"] = np.array(sorted(gs))
                 keep = {"aq_embed": aq_embed, "mq_embed": mq_embed}
+                if cfg.get("embed_samples"):
+                    rows = embed_rows(cfg["B"], cfg["embed_samples"])
+                    blob["embed_rows"] = rows
+                    keep = {k: v[torch.from_numpy(rows)] for k, v in keep.items()}
                 if cfg["full"]:
                     for i in range(len(aq)):
                         keep.update({f"com_app_{i}": ca[i], f"com_mot_{i}": cm[i], f"aq_fusion_{i}": aq[i],

@@ -141,7 +141,8 @@ def test_fp32_mode_against_reference_golden(golden, fp32_mode, name):
     e_log = rel(out[0], ref_logits)
     assert e_log < TOL32, e_log
     assert np.array_equal(out[0].argmax(1).cpu().numpy(), ref_logits.argmax(1))
-    assert rel(out[1], g["f64_aq_embed"]) < TOL32 and rel(out[2], g["f64_mq_embed"]) < TOL32
+    rows = g["embed_rows"] if "embed_rows" in g.files else slice(None)     # g4 keeps a seeded subset of the batch
+    assert rel(out[1][rows], g["f64_aq_embed"]) < TOL32 and rel(out[2][rows], g["f64_mq_embed"]) < TOL32
     if "f64_com_app_0" in g.files:
         for i in range(len(out[3])):
             for key, lst in (("com_app", out[3]), ("com_mot", out[4]), ("aq_fusion", out[5]), ("mq_fusion", out[6])):

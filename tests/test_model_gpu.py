@@ -83,7 +83,8 @@ def test_against_reference_golden(golden, name):
           f"rows whose top-2 margin exceeds the tolerance: {int(confident.sum())}")
     # a flip is only tolerated on a row the reference itself decides by less than the stated tolerance (asserted above)
     assert agree >= len(got_arg) - int((~confident).sum())
-    assert rel(out[1], g["f64_aq_embed"]) < TOL and rel(out[2], g["f64_mq_embed"]) < TOL
+    rows = g["embed_rows"] if "embed_rows" in g.files else slice(None)     # g4 keeps a seeded subset of the batch
+    assert rel(out[1][rows], g["f64_aq_embed"]) < TOL and rel(out[2][rows], g["f64_mq_embed"]) < TOL
     if "f64_com_app_0" in g.files:
         for i in range(len(out[3])):
             for key, lst in (("com_app", out[3]), ("com_mot", out[4]), ("aq_fusion", out[5]), ("mq_fusion", out[6])):

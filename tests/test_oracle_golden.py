@@ -61,8 +61,9 @@ def test_forward_train_losses_and_grads_match_reference(golden, name):
     logits = out[0]
     assert _rel(logits.detach().numpy(), g["f64_logits_train"]) < 1e-9
     assert np.array_equal(logits.detach().numpy().argmax(1), g["f64_logits_train"].argmax(1))
-    assert _rel(out[1].detach().numpy(), g["f64_aq_embed"]) < 1e-6      # fixture stores float32
-    assert _rel(out[2].detach().numpy(), g["f64_mq_embed"]) < 1e-6
+    rows = g["embed_rows"] if "embed_rows" in g.files else slice(None)     # g4 keeps a seeded subset of the batch
+    assert _rel(out[1].detach().numpy()[rows], g["f64_aq_embed"]) < 1e-6      # fixture stores float32
+    assert _rel(out[2].detach().numpy()[rows], g["f64_mq_embed"]) < 1e-6
     if "f64_com_app_0" in g.files:
         for i in range(len(out[3])):
             for key, lst in (("com_app", out[3]), ("com_mot", out[4]), ("aq_fusion", out[5]), ("mq_fusion", out[6])):
