@@ -148,6 +148,8 @@ aux_loss_unit = _sig("dvgr_aux_loss_unit", [P, P, P, P, c_float, c_float, c_int,
 aux_loss_unit_ex = _sig("dvgr_aux_loss_unit_ex", [P, P, P, P, c_float, c_float, c_int, c_int, c_int, P, P, P, P, P, P, c_int, P])
 prep_features = _sig("dvgr_prep_features", [P, P, c_ll, c_int, c_int, c_int, c_int, c_float, c_ull, c_uint, P])
 prep_features_ex = _sig("dvgr_prep_features_ex", [P, c_int, P, c_ll, c_int, c_int, c_int, c_int, c_float, c_ull, c_uint, P])
+prep_features_gather = _sig("dvgr_prep_features_gather", [P, c_int, c_ll, c_int, P, c_int, P, c_int, c_int, c_int, c_int,
+                                                           c_float, c_ull, c_uint, P, P])
 cast_rows = _sig("dvgr_cast_rows", [P, c_ll, P, c_ll, c_int, c_int, c_int, c_int, P])
 dropout = _sig("dvgr_dropout", [P, P, c_ll, c_float, c_ull, c_uint, P])
 act_bwd = _sig("dvgr_act_bwd", [P, P, P, c_ll, c_int, c_int, c_float, c_ull, c_uint, P])
@@ -202,7 +204,7 @@ lstm32_cell_bwd = _sig("dvgr_lstm32_cell_bwd", [ctypes.POINTER(Lstm32Args), P])
 # entry point below under the suffix _f32 with an identical signature (every bf16 activation pointer is a float pointer)
 F32_VARIANTS = ["gat_attn_fwd", "gat_attn_bwd", "qattn_fwd", "qattn_bwd", "gate_fwd", "gate_bwd", "view_attn_fwd",
                 "view_attn_bwd", "mfb_fwd", "mfb_bwd", "readout_fwd", "readout_bwd", "bn_fwd_ex", "bn_bwd_ex",
-                "prep_features_ex", "dropout", "act_bwd", "add", "embed_fwd", "embed_bwd"]
+                "prep_features_ex", "prep_features_gather", "dropout", "act_bwd", "add", "embed_fwd", "embed_bwd"]
 for _n in F32_VARIANTS:
     globals()[_n + "_f32"] = _sig("dvgr_" + _n + "_f32", list(globals()[_n].argtypes))
 
@@ -217,7 +219,7 @@ EXPORTED = [
     "dvgr_lstm_step_fwd", "dvgr_lstm_step_bwd", "dvgr_lstm_seq_fwd", "dvgr_lstm_seq_sync_words", "dvgr_lstm_seq_bwd", "dvgr_gat_attn_fwd", "dvgr_gat_attn_bwd", "dvgr_qattn_fwd",
     "dvgr_qattn_bwd", "dvgr_gate_fwd", "dvgr_gate_bwd", "dvgr_view_attn_fwd", "dvgr_view_attn_bwd_blocks",
     "dvgr_view_attn_bwd", "dvgr_mfb_fwd", "dvgr_mfb_bwd", "dvgr_readout_fwd", "dvgr_readout_bwd", "dvgr_bn_fwd",
-    "dvgr_bn_bwd", "dvgr_cross_entropy", "dvgr_pair_loss_workspace", "dvgr_pair_loss_multi", "dvgr_aux_loss_workspace", "dvgr_aux_loss_unit", "dvgr_aux_loss_unit_ex", "dvgr_prep_features", "dvgr_prep_features_ex", "dvgr_cast_rows", "dvgr_dropout",
+    "dvgr_bn_bwd", "dvgr_cross_entropy", "dvgr_pair_loss_workspace", "dvgr_pair_loss_multi", "dvgr_aux_loss_workspace", "dvgr_aux_loss_unit", "dvgr_aux_loss_unit_ex", "dvgr_prep_features", "dvgr_prep_features_ex", "dvgr_prep_features_gather", "dvgr_cast_rows", "dvgr_dropout",
     "dvgr_act_bwd", "dvgr_add", "dvgr_scatter", "dvgr_colsum_workspace", "dvgr_colsum", "dvgr_colsum_batched", "dvgr_colsum_grouped", "dvgr_sumsq_blocks", "dvgr_sumsq",
     "dvgr_adam_step", "dvgr_dropout_multi", "dvgr_gat_input_bwd", "dvgr_embed_fwd", "dvgr_embed_bwd",
     "dvgr_view_attn_fwd_multi", "dvgr_view_attn_bwd_multi", "dvgr_cast_rows_grouped", "dvgr_lstm_pack_bias",

@@ -425,13 +425,21 @@ class AppearanceEncoderFn(Function):
     input-to-hidden product of both directions (N = 8H), T fused recurrent steps, final dropout."""
 
     @staticmethod
-    def forward(ctx, app, w_ih, w_hh, b_ih, b_hh, w_ih_r, w_hh_r, b_ih_r, b_hh_r, p_in, p_out, training, out_slot=None):
+    def forward(ctx, app, w_ih, w_hh, b_ih, b_hh, w_ih_r, w_hh_r, b_ih_r, b_hh_r, p_in, p_out, training, out_slot=None,
+                rows=None, err=None):
         """out_slot: optional 1-tuple holding a preallocated [B*N, 2H] bf16 buffer for the result (the unit stack carries
-        the appearance and motion streams as ONE [2, B*N, D] tensor: its producers write straight into the halves)."""
-        B, N, T, Dv = app.shape
+        the appearance and motion streams as ONE [2, B*N, D] tensor: its producers write straight into the halves).
+        rows: optional [B] int32 video rows; app is then a device-resident store [V, N, F, Dv] and the prologue reads the
+        batch app[rows] from it (err: the store's sticky out-of-range word)."""
+        _, N, T, Dv = app.shape
+        B = app.shape[0] if rows is None else rows.numel()
         S, H = B * N, w_hh.shape[1]
         seed, sid = _site(2)
-        xa = ops.prep_features(_c(app).view(S * T, Dv), T, True, True, p_in if training else 0.0, seed, sid)
+        p_x = p_in if training else 0.0
+        if rows is None:
+            xa = ops.prep_features(_c(app).view(S * T, Dv), T, True, True, p_x, seed, sid)
+        else:
+            xa = ops.prep_features_gather(app, rows, T, True, True, p_x, seed, sid, err)
         wih = _lstm_weight([w_ih, w_ih_r], H, "ih")
         whh = _lstm_weight([w_hh, w_hh_r], H, "hh").view(2, 4 * H, H)
         bias = ops.lstm_pack_bias([b_ih.detach(), b_ih_r.detach()], [b_hh.detach(), b_hh_r.detach()], H)
@@ -515,7 +523,7 @@ class AppearanceEncoderFn(Function):
         g_ih = (None, None) if dwih is None else (dwih[:4 * H], dwih[4 * H:])
         g_hh = (None, None) if t_hh is not None else (dwhh[0], dwhh[1])
         # b_ih, b_hh, b_ih_reverse, b_hh_reverse: both biases of a direction get the same gradient
-        return (None, g_ih[0], g_hh[0], dbs[0], dbs[1], g_ih[1], g_hh[1], dbs[2], dbs[3], None, None, None, None)
+        return (None, g_ih[0], g_hh[0], dbs[0], dbs[1], g_ih[1], g_hh[1], dbs[2], dbs[3], None, None, None, None, None, None)
 
 
 def _lstm_weight(params, H, tag):

@@ -569,23 +569,60 @@ __device__ __forceinline__ void prep_item(const TIN* __restrict__ in, bf16* __re
   store8(out + o * 8, f);
 }
 
-template <typename TIN>
+// Gathered input (GATHER): `in` is a feature store [V][N][T][C] resident in device memory and batch item b is video
+// rows[b]; everything else (item index i, output layout, dropout mask keyed by i) is that of the dense pass over the
+// batch store[rows]. The batch side keeps 32-bit index arithmetic; the store offset rows[b]*N*T*C is 64-bit (a store
+// passes 2^31 elements at ~3300 SVQA videos). A row outside [0, V) is never read: its items are zeros (tanh(0) = 0, so its
+// output rows are zero) and the sticky word *err is set.
+struct GatherCfg {
+  const int* rows;
+  long long V;
+  int slab8;      // N * T * C / 8: 8-element items per video
+  int* err;
+};
+
+template <typename TIN, bool GATHER>
+__device__ __forceinline__ void prep_load(const TIN* __restrict__ in, long long i, float (&f)[8], const GatherCfg& g) {
+  if constexpr (!GATHER) {
+    load8g(in + i * 8, f);
+  } else {
+    long long b, w;
+    if (i < 0x7fffffffLL) {
+      const unsigned iu = (unsigned)i, bu = iu / (unsigned)g.slab8;
+      b = bu;
+      w = iu - bu * (unsigned)g.slab8;
+    } else {
+      b = i / g.slab8;
+      w = i - b * g.slab8;
+    }
+    const int r = __ldg(g.rows + b);
+    if (r < 0 || r >= g.V) {
+#pragma unroll
+      for (int q = 0; q < 8; ++q) f[q] = 0.f;
+      *g.err = 1;
+      return;
+    }
+    load8g(in + ((long long)r * g.slab8 + w) * 8, f);
+  }
+}
+
+template <typename TIN, bool GATHER>
 __global__ void prep_features_kernel(const TIN* __restrict__ in, bf16* __restrict__ out, long long S, int T, int C,
-                                     int do_tanh, int time_major, DropoutCfg dc) {
+                                     int do_tanh, int time_major, DropoutCfg dc, GatherCfg g) {
   const long long n8 = S * T * (long long)C / 8;
   const int c8 = C / 8;
   const long long stride = (long long)gridDim.x * blockDim.x;
   long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
   for (; i + stride < n8; i += 2 * stride) {      // two items per trip: both loads are in flight before either is consumed
     float f0[8], f1[8];
-    load8g(in + i * 8, f0);
-    load8g(in + (i + stride) * 8, f1);
+    prep_load<TIN, GATHER>(in, i, f0, g);
+    prep_load<TIN, GATHER>(in, i + stride, f1, g);
     prep_item<TIN>(in, out, i, f0, S, T, c8, do_tanh, time_major, dc);
     prep_item<TIN>(in, out, i + stride, f1, S, T, c8, do_tanh, time_major, dc);
   }
   if (i < n8) {
     float f0[8];
-    load8g(in + i * 8, f0);
+    prep_load<TIN, GATHER>(in, i, f0, g);
     prep_item<TIN>(in, out, i, f0, S, T, c8, do_tanh, time_major, dc);
   }
 }
@@ -1172,12 +1209,36 @@ extern "C" int DVGR_FN(dvgr_prep_features_ex)(const void* in, int in_is_bf16, vo
   const long long n = S * T * (long long)C / 8;
   if (n <= 0) return 0;
   DropoutCfg dc{seed, drop_stream, p, seed_offset_ptr()};
+  const GatherCfg g{nullptr, 0, 0, nullptr};
   if (in_is_bf16)
-    prep_features_kernel<__nv_bfloat16><<<grid_for(n, 256, 148 * 32), 256, 0, ST(stream)>>>(reinterpret_cast<const __nv_bfloat16*>(in), BF(out), S, T, C, do_tanh, time_major, dc);
+    prep_features_kernel<__nv_bfloat16, false><<<grid_for(n, 256, 148 * 32), 256, 0, ST(stream)>>>(reinterpret_cast<const __nv_bfloat16*>(in), BF(out), S, T, C, do_tanh, time_major, dc, g);
   else
-    prep_features_kernel<float><<<grid_for(n, 256, 148 * 32), 256, 0, ST(stream)>>>(reinterpret_cast<const float*>(in), BF(out), S, T, C,
-                                                                                    do_tanh, time_major, dc);
+    prep_features_kernel<float, false><<<grid_for(n, 256, 148 * 32), 256, 0, ST(stream)>>>(reinterpret_cast<const float*>(in), BF(out), S, T, C,
+                                                                                    do_tanh, time_major, dc, g);
   DVGR_CHECK_LAUNCH("prep_features");
+  return 0;
+}
+
+extern "C" int DVGR_FN(dvgr_prep_features_gather)(const void* store, int store_is_bf16, long long V, int N, const int* rows,
+                                                  int B, void* out, int T, int C, int do_tanh, int time_major, float p,
+                                                  unsigned long long seed, unsigned int drop_stream, int* err, void* stream) {
+  if (C % 8 != 0) return set_error("prep_features_gather: C=%d must be a multiple of 8", C);
+  if (V < 0 || N <= 0 || T <= 0 || B < 0) return set_error("prep_features_gather: V=%lld N=%d T=%d B=%d", V, N, T, B);
+  if (!store || !rows || !out || !err) return set_error("prep_features_gather: null buffer");
+  const long long slab8 = (long long)N * T * (C / 8);
+  if (slab8 > 0x7fffffffLL) return set_error("prep_features_gather: N*T*C/8=%lld exceeds 2^31", slab8);
+  const long long S = (long long)B * N;
+  const long long n = S * T * (long long)C / 8;
+  if (n <= 0) return 0;
+  DropoutCfg dc{seed, drop_stream, p, seed_offset_ptr()};
+  const GatherCfg g{rows, V, (int)slab8, err};
+  if (store_is_bf16)
+    prep_features_kernel<__nv_bfloat16, true><<<grid_for(n, 256, 148 * 32), 256, 0, ST(stream)>>>(
+        reinterpret_cast<const __nv_bfloat16*>(store), BF(out), S, T, C, do_tanh, time_major, dc, g);
+  else
+    prep_features_kernel<float, true><<<grid_for(n, 256, 148 * 32), 256, 0, ST(stream)>>>(
+        reinterpret_cast<const float*>(store), BF(out), S, T, C, do_tanh, time_major, dc, g);
+  DVGR_CHECK_LAUNCH("prep_features_gather");
   return 0;
 }
 

@@ -22,6 +22,7 @@ import torch.distributed as dist
 from . import autograd as ag
 from . import fused_stack as fs
 from . import ops
+from .loader import DeviceFeatureStore
 
 _LIVE_ENGINES = weakref.WeakSet()
 
@@ -199,9 +200,30 @@ class TrainEngine:
         """Forward, losses, backward of this rank's shard: leaves the (unreduced) gradient in gflat and the step's statistics
         in last_stats. Returns (total loss (device scalar), n_correct [B] int32)."""
         with self._on_stream():
-            return self._forward_backward(app, mot, question, question_len, answers)
+            return self._forward_backward((app, mot), question, question_len, answers)
 
-    def _forward_backward_fp32(self, app, mot, question, question_len, answers):
+    @staticmethod
+    def _run_model(model, feats, question, question_len):
+        """feats: (app, mot) dense batches, or (DeviceFeatureStore, rows) -> the model's 7-tuple."""
+        src, x = feats
+        if isinstance(src, DeviceFeatureStore):
+            return model.forward_from_store(src, x, question, question_len)
+        return model(src, x, question, question_len)
+
+    @staticmethod
+    def _batch_dims(feats):
+        """(B, N, device) of the batch that feats describes (see _run_model)."""
+        src, x = feats
+        if isinstance(src, DeviceFeatureStore):
+            return x.shape[0], src.app.shape[1], x.device
+        return src.shape[0], src.shape[1], src.device
+
+    @staticmethod
+    def _store_flags(feats):
+        """The store's sticky out-of-range word joins the step flags: a step that read a bad row finalises to NaN."""
+        return [feats[0].err] if isinstance(feats[0], DeviceFeatureStore) else []
+
+    def _forward_backward_fp32(self, feats, question, question_len, answers):
         """fp32 mode (DualVGR.set_precision("fp32")): module-by-module forward, the auxiliary terms as ordinary autograd nodes
         on the fp32 graph outputs, gradients accumulated by autograd into the bound views of gflat (no deferred launches)."""
         model = self.model
@@ -209,8 +231,8 @@ class TrainEngine:
         self.gflat.zero_()
         ag.begin_step_flags()
         unit = model.visual_input_unit
-        B, N = app.shape[0], app.shape[1]
-        outputs = model(app, mot, question, question_len)
+        B, N, _ = self._batch_dims(feats)
+        outputs = self._run_model(model, feats, question, question_len)
         self.last_logits = outputs[0].detach()
         ce, correct = ag.CrossEntropyFn.apply(outputs[0], answers, False)
         loss, parts = ce, []
@@ -221,35 +243,37 @@ class TrainEngine:
                 loss = loss + tot
                 parts.append(vals)
         loss.backward()
-        self.last_stats = ops.finalize_loss(ce.detach().reshape(1), torch.stack(parts) if parts else None, [])
+        self.last_stats = ops.finalize_loss(ce.detach().reshape(1), torch.stack(parts) if parts else None,
+                                            self._store_flags(feats))
         return self.last_stats[0], correct
 
-    def _forward_backward(self, app, mot, question, question_len, answers):
+    def _forward_backward(self, feats, question, question_len, answers):
+        """feats: (app, mot) or (DeviceFeatureStore, rows), see _run_model."""
         if ag.ACT[0] == torch.float32:
-            return self._forward_backward_fp32(app, mot, question, question_len, answers)
+            return self._forward_backward_fp32(feats, question, question_len, answers)
         model = self.model
         model.train()
+        B, N, dev = self._batch_dims(feats)
         # the 122 MB gradient buffer is cleared on a side stream, under the forward pass (nothing writes it before backward)
         cur = torch.cuda.current_stream()
-        zs = fs.side_stream(app.device, "aux")
+        zs = fs.side_stream(dev, "aux")
         zs.wait_stream(cur)
         with torch.cuda.stream(zs):
             self.gflat.zero_()
             ev_zero = torch.cuda.Event()
             ev_zero.record()
         ag.begin_step_flags()
-        ops.begin_step_counters(app.device)        # zeroed tile counters of this step's dynamically scheduled GEMMs
+        ops.begin_step_counters(dev)               # zeroed tile counters of this step's dynamically scheduled GEMMs
         unit = model.visual_input_unit
-        B, N = app.shape[0], app.shape[1]
         if self._reserve_env is None:
             ops.RESERVE_SMS[0] = min(64, 4 * ((B + 31) // 32))
         parts = None
         if unit.layers > 0 and (self.alpha != 0 or self.beta != 0):
             c_com, c_dep = self._loss_coefs(B, N, unit.layers)
-            parts = torch.empty((unit.layers, B, 3), dtype=torch.float32, device=app.device)
+            parts = torch.empty((unit.layers, B, 3), dtype=torch.float32, device=dev)
             unit._aux = (c_com, c_dep, parts)
         try:
-            outputs = model(app, mot, question, question_len)
+            outputs = self._run_model(model, feats, question, question_len)
         finally:
             unit._aux = None
         self.last_logits = outputs[0].detach()
@@ -263,9 +287,10 @@ class TrainEngine:
             raise
         finally:
             ops.DEFER_WGRAD[0] = False
-        ops.end_step_counters(app.device)
-        fs.join_side_streams(app.device)   # question-encoder backward / auxiliary losses ran on side streams
+        ops.end_step_counters(dev)
+        fs.join_side_streams(dev)          # question-encoder backward / auxiliary losses ran on side streams
         ops.flush_wgrads()                 # ... and launched as ONE grouped tcgen05 GEMM + grouped column sums
+        ag._STEP_FLAGS.extend(self._store_flags(feats))
         self.last_stats = ops.finalize_loss(ce.detach(), parts, ag.step_flags())
         return self.last_stats[0], correct
 
@@ -284,7 +309,17 @@ class TrainEngine:
         """One optimizer step on this rank's shard. Returns the (device) total loss of the shard."""
         self._last_BN = (app.shape[0], app.shape[1])
         with self._on_stream():
-            total, _ = self._forward_backward(app, mot, question, question_len, answers)
+            total, _ = self._forward_backward((app, mot), question, question_len, answers)
+            self._optimizer_step()
+        return total
+
+    def train_step_from_store(self, dstore, rows, question, question_len, answers):
+        """train_step() on the batch (dstore.app[rows], dstore.mot[rows]) of a device-resident feature store
+        (loader.DeviceFeatureStore), gathered inside the input prologue kernels. rows [B] int32 on the device. A row
+        outside [0, V) sets dstore.err, and while that word is set every step's loss is NaN."""
+        self._last_BN = (rows.shape[0], dstore.app.shape[1])
+        with self._on_stream():
+            total, _ = self._forward_backward((dstore, rows), question, question_len, answers)
             self._optimizer_step()
         return total
 
@@ -312,8 +347,9 @@ class TrainEngine:
         ag.invalidate_weight_cache()
 
     def dependency_poll_timeouts(self):
-        """Number of LSTM dependency polls that gave up in the last step, max over ranks (0 in a healthy run; a non-zero
-        value also turned that step's loss into NaN). Synchronises."""
+        """Number of step flags that were set in the last step, max over ranks: LSTM dependency polls that gave up and, in a
+        step fed from a DeviceFeatureStore, the store's out-of-range-row word (0 in a healthy run; a non-zero value also
+        turned that step's loss into NaN). Synchronises."""
         t = torch.zeros(1, device=self.flat.device) if self.last_stats is None else self.last_stats[3:4].clone()
         if self.world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX, group=self.pg)
@@ -329,18 +365,28 @@ class TrainEngine:
         input buffers; afterwards: load_batch(...) + replay(). NOTE: the `warmup` eager steps that precede the capture are
         REAL optimizer steps on the given batch (they warm the allocator, the weight caches and the side streams); pass the
         first training batch, or warmup=0 after at least one eager train_step()."""
+        def step(st):
+            return self.train_step(st["app"], st["mot"], st["q"], st["qlen"], st["ans"])
+        return self._capture(dict(app=app, mot=mot, q=question, qlen=question_len, ans=answers), step, warmup)
+
+    def capture_from_store(self, dstore, rows, question, question_len, answers, warmup=3):
+        """capture() for train_step_from_store: the graph's static inputs are the rows and the question / answer tensors
+        only (no feature buffers); afterwards load_rows(...) + replay(). The `warmup` eager steps are real optimizer steps."""
+        def step(st):
+            return self.train_step_from_store(dstore, st["rows"], st["q"], st["qlen"], st["ans"])
+        return self._capture(dict(rows=rows, q=question, qlen=question_len, ans=answers), step, warmup)
+
+    def _capture(self, named, step, warmup):
         from . import _lib
-        self.static = {k: torch.empty_like(v) for k, v in
-                       dict(app=app, mot=mot, q=question, qlen=question_len, ans=answers).items()}
-        for k, v in dict(app=app, mot=mot, q=question, qlen=question_len, ans=answers).items():
+        self.static = {k: torch.empty_like(v) for k, v in named.items()}
+        for k, v in named.items():
             self.static[k].copy_(v)
         _lib.lib.dvgr_set_seed_offset(self.seed_dev.data_ptr())
         self._seed_owner = True
 
         def body():
             self.seed_dev += 1
-            st = self.static
-            return self.train_step(st["app"], st["mot"], st["q"], st["qlen"], st["ans"])
+            return step(self.static)
 
         side = self.stream
         side.wait_stream(torch.cuda.current_stream())
@@ -385,6 +431,12 @@ class TrainEngine:
     def load_batch(self, app, mot, question, question_len, answers, non_blocking=True):
         st = self.static
         for k, v in dict(app=app, mot=mot, q=question, qlen=question_len, ans=answers).items():
+            st[k].copy_(v, non_blocking=non_blocking)
+
+    def load_rows(self, rows, question, question_len, answers, non_blocking=True):
+        """The next batch of a capture_from_store() graph: B video rows (int32) and the question / answer tensors."""
+        st = self.static
+        for k, v in dict(rows=rows, q=question, qlen=question_len, ans=answers).items():
             st[k].copy_(v, non_blocking=non_blocking)
 
     def replay(self):

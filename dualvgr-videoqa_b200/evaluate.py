@@ -41,7 +41,19 @@ class EvalEngine:
     def step(self, app, mot, question, question_len, answers, question_categories=None, want_preds=False):
         """One validation batch: returns (logits, preds | None); the counters accumulate on the device."""
         self.model.eval()
-        logits = self.model(app, mot, question, question_len)[0]
+        return self._count(self.model(app, mot, question, question_len)[0], question, answers, question_categories,
+                           want_preds)
+
+    @torch.no_grad()
+    def step_from_store(self, dstore, rows, question, question_len, answers, question_categories=None, want_preds=False):
+        """step() on the batch (dstore.app[rows], dstore.mot[rows]) of a device-resident feature store
+        (loader.DeviceFeatureStore), gathered inside the input prologue kernels; rows [B] int32 on the device. A row
+        outside [0, V) sets dstore.err (read it with dstore.read_error())."""
+        self.model.eval()
+        return self._count(self.model.forward_from_store(dstore, rows, question, question_len)[0], question, answers,
+                           question_categories, want_preds)
+
+    def _count(self, logits, question, answers, question_categories, want_preds):
         preds = ops.accuracy_counters(logits, answers.reshape(-1), self.counts,
                                       category=question_categories.reshape(-1) if question_categories is not None else None,
                                       tokens=question if (question_categories is None and self.token_to_cat is not None) else None,
@@ -50,7 +62,19 @@ class EvalEngine:
 
     def capture(self, app, mot, question, question_len, answers, question_categories=None):
         """Records the eval step as a CUDA graph over static input buffers (load_batch + replay afterwards)."""
-        named = dict(app=app, mot=mot, q=question, qlen=question_len, ans=answers)
+        def step(st):
+            return self.step(st["app"], st["mot"], st["q"], st["qlen"], st["ans"], st.get("cat"))
+        return self._capture(dict(app=app, mot=mot, q=question, qlen=question_len, ans=answers), question_categories, step)
+
+    def capture_from_store(self, dstore, rows, question, question_len, answers, question_categories=None):
+        """capture() for step_from_store: static inputs are the rows and the question / answer (/ category) tensors only;
+        load_rows + replay afterwards. The graph has the batch size of `rows`: run a shorter last batch through
+        step_from_store."""
+        def step(st):
+            return self.step_from_store(dstore, st["rows"], st["q"], st["qlen"], st["ans"], st.get("cat"))
+        return self._capture(dict(rows=rows, q=question, qlen=question_len, ans=answers), question_categories, step)
+
+    def _capture(self, named, question_categories, step):
         if question_categories is not None:
             named["cat"] = question_categories
         self.static = {k: v.clone() for k, v in named.items()}
@@ -60,18 +84,25 @@ class EvalEngine:
         saved = self.counts.clone()
         with torch.cuda.stream(side):
             for _ in range(2):
-                self.step(st["app"], st["mot"], st["q"], st["qlen"], st["ans"], st.get("cat"))
+                step(st)
         torch.cuda.current_stream().wait_stream(side)
         torch.cuda.synchronize()
         self.graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(self.graph):
-            self.static_logits, _ = self.step(st["app"], st["mot"], st["q"], st["qlen"], st["ans"], st.get("cat"))
+            self.static_logits, _ = step(st)
         self.counts.copy_(saved)                      # warm-up and capture must not count
         return self.graph
 
     def load_batch(self, **tensors):
         for k, v in tensors.items():
             self.static[k].copy_(v, non_blocking=True)
+
+    def load_rows(self, rows, question, question_len, answers, question_categories=None):
+        """The next full batch of a capture_from_store() graph."""
+        named = dict(rows=rows, q=question, qlen=question_len, ans=answers)
+        if question_categories is not None:
+            named["cat"] = question_categories
+        self.load_batch(**named)
 
     def replay(self):
         self.graph.replay()

@@ -104,12 +104,15 @@ class VisualAppearanceEncoder(nn.Module):
         self.embedding_dropout = nn.Dropout(p=0.15)
         self.finalvisual_dropout = nn.Dropout(p=0.18)
 
-    def forward(self, appearance_clips, out=None):
+    def forward(self, appearance_clips, out=None, rows=None, err=None):
         """[B, N, F, Dv] fp32 -> [B, N, module_dim] bf16 (final forward / backward hidden states, concatenated).
-        out: optional preallocated [B*N, module_dim] bf16 buffer for the result."""
+        out: optional preallocated [B*N, module_dim] bf16 buffer for the result.
+        rows: optional [B] int32 video rows; appearance_clips is then a device-resident store [V, N, F, Dv] (fp32 / bf16)
+        read at those rows inside the prologue (err: its sticky [1] int32 out-of-range word, loader.DeviceFeatureStore)."""
         e = self.encoder
         x = appearance_clips if appearance_clips.dtype == torch.bfloat16 else appearance_clips.float()   # bf16-stored features pass through
         return ag.AppearanceEncoderFn.apply(
             x, e.weight_ih_l0, e.weight_hh_l0, e.bias_ih_l0, e.bias_hh_l0,
             e.weight_ih_l0_reverse, e.weight_hh_l0_reverse, e.bias_ih_l0_reverse, e.bias_hh_l0_reverse,
-            self.embedding_dropout.p, self.finalvisual_dropout.p, self.training, (out,) if out is not None else None)
+            self.embedding_dropout.p, self.finalvisual_dropout.p, self.training, (out,) if out is not None else None,
+            rows, err)

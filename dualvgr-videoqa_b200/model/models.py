@@ -68,12 +68,14 @@ class DualVGR(nn.Module):
         ag.ACT[0] = torch.float32 if precision == "fp32" else BF16
         return self
 
-    def _forward_fp32(self, video_appearance_feat, video_motion_feat, question, question_len):
-        """fp32 mode: module-by-module, fp32 activations (fp32_path.py). Same returns as forward()."""
+    def _forward_fp32(self, video_appearance_feat, video_motion_feat, question, question_len, rows=None, err=None):
+        """fp32 mode: module-by-module, fp32 activations (fp32_path.py). Same returns as forward(). With rows, the two
+        feature arguments are device-resident stores read at those rows (forward_from_store)."""
         from dualvgr_videoqa_b200 import fp32_path as f32
         ag.begin_forward()
         training = self.training
-        B, N, T, Dv = video_appearance_feat.shape
+        _, N, T, Dv = video_appearance_feat.shape
+        B = video_appearance_feat.shape[0] if rows is None else rows.numel()
         D = self.visual_motion_input_unit.out_features
         qlen = question_len.to(torch.int32)
         lin = self.linguistic_input_unit
@@ -84,15 +86,23 @@ class DualVGR(nn.Module):
         question_embedding = ag.dropout(last[:, D:], lin.final_dropout.p, training)
         enc = self.visual_appearance_input_unit
         seed, sid = ag._site()
-        feats = video_appearance_feat if video_appearance_feat.dtype == BF16 else video_appearance_feat.float()
-        xa = ag.ops.prep_features(feats.contiguous().view(B * N * T, Dv), T, True, True,
-                                  enc.embedding_dropout.p if training else 0.0, seed, sid, out_dtype=torch.float32)
+        p_x = enc.embedding_dropout.p if training else 0.0
+        if rows is None:
+            feats = video_appearance_feat if video_appearance_feat.dtype == BF16 else video_appearance_feat.float()
+            xa = ag.ops.prep_features(feats.contiguous().view(B * N * T, Dv), T, True, True, p_x, seed, sid,
+                                      out_dtype=torch.float32)
+        else:
+            xa = ag.ops.prep_features_gather(video_appearance_feat, rows, T, True, True, p_x, seed, sid, err,
+                                             out_dtype=torch.float32)
         e = enc.encoder
         _, h = f32.Lstm32Fn.apply(xa.view(T, B * N, Dv), None, False, e.weight_ih_l0, e.weight_hh_l0, e.bias_ih_l0, e.bias_hh_l0,
                                   e.weight_ih_l0_reverse, e.weight_hh_l0_reverse, e.bias_ih_l0_reverse, e.bias_hh_l0_reverse)
         app = ag.dropout(h, enc.finalvisual_dropout.p, training).view(B, N, D)
-        mot = ag.linear(video_motion_feat.float().contiguous().view(B * N, Dv), self.visual_motion_input_unit.weight,
-                        self.visual_motion_input_unit.bias).view(B, N, D)
+        if rows is None:
+            mot_in = video_motion_feat.float().contiguous().view(B * N, Dv)
+        else:
+            mot_in = ag.ops.prep_features_gather(video_motion_feat, rows, 1, False, False, err=err, out_dtype=torch.float32)
+        mot = ag.linear(mot_in, self.visual_motion_input_unit.weight, self.visual_motion_input_unit.bias).view(B, N, D)
         visual, aq_embed, mq_embed, com_app, com_motion, aq_fusion, mq_fusion = self.visual_input_unit(
             app, mot, dynamic_q, words, qlen)
         pooled = self.feature_aggregation(visual)
@@ -107,11 +117,25 @@ class DualVGR(nn.Module):
         """
         if not video_appearance_feat.is_cuda:
             raise RuntimeError("dualvgr_b200: DualVGR runs on sm_100a CUDA devices only; there is no CPU path")
+        return self._forward(video_appearance_feat, video_motion_feat, question, question_len)
+
+    def forward_from_store(self, dstore, rows, question, question_len):
+        """forward() on the batch (dstore.app[rows], dstore.mot[rows]) of a device-resident feature store
+        (loader.DeviceFeatureStore), read inside the two input prologue kernels: no batch of clip features is copied.
+        rows [B] int32 on the store's device. Same returns as forward(), bit for bit. A row outside [0, V) reads zeros and
+        sets dstore.err."""
+        if not rows.is_cuda:
+            raise RuntimeError("dualvgr_b200: DualVGR runs on sm_100a CUDA devices only; there is no CPU path")
+        return self._forward(dstore.app, dstore.mot, question, question_len, rows, dstore.err)
+
+    def _forward(self, video_appearance_feat, video_motion_feat, question, question_len, rows=None, err=None):
+        """Body of forward() / forward_from_store(): only the two input prologues differ (rows None: dense batches)."""
         if ag.ACT[0] == torch.float32:
-            return self._forward_fp32(video_appearance_feat, video_motion_feat, question, question_len)
+            return self._forward_fp32(video_appearance_feat, video_motion_feat, question, question_len, rows, err)
         ag.begin_forward()
         dev = video_appearance_feat.device
-        B, N = video_motion_feat.shape[:2]
+        N = video_motion_feat.shape[1]
+        B = video_motion_feat.shape[0] if rows is None else rows.numel()
         D = self.visual_motion_input_unit.out_features
         qlen = question_len.to(torch.int32)
         # question encoder on a (high-priority) side stream: two 20-step recurrences over 256 sequences keep ~1/3 of the SMs
@@ -128,9 +152,12 @@ class DualVGR(nn.Module):
             chain = self.visual_input_unit.launch_query_chain(launched[1])
         # the two clip streams are carried as ONE stacked [2, B*N, D] tensor: both encoders write into its halves
         x0 = torch.empty((2, B * N, D), dtype=BF16, device=dev)
-        app = self.visual_appearance_input_unit(video_appearance_feat, out=x0[0])
-        mf = video_motion_feat if video_motion_feat.dtype == torch.bfloat16 else video_motion_feat.float()
-        mot_in = ag.ops.prep_features(mf.contiguous().view(B * N, -1), 1, False, False)
+        app = self.visual_appearance_input_unit(video_appearance_feat, out=x0[0], rows=rows, err=err)
+        if rows is None:
+            mf = video_motion_feat if video_motion_feat.dtype == torch.bfloat16 else video_motion_feat.float()
+            mot_in = ag.ops.prep_features(mf.contiguous().view(B * N, -1), 1, False, False)
+        else:
+            mot_in = ag.ops.prep_features_gather(video_motion_feat, rows, 1, False, False, err=err)
         mot = ag.linear(mot_in, self.visual_motion_input_unit.weight, self.visual_motion_input_unit.bias, out=x0[1]).view(B, N, D)
         with torch.cuda.stream(side):
             question_embedding, word_embedding, dynamic_q = self.linguistic_input_unit.fused(question, qlen, launched)

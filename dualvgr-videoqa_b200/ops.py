@@ -495,6 +495,25 @@ def prep_features(x, T, do_tanh, time_major, p=0.0, seed=0, stream_id=0, out_dty
     return out
 
 
+def prep_features_gather(store, rows, T, do_tanh, time_major, p=0.0, seed=0, stream_id=0, err=None, out_dtype=BF16):
+    """prep_features of the batch store[rows] read straight from a device-resident store: store [V, N, T, C] (or [V, N, C]
+    with T = 1) fp32 / bf16, rows [B] int32 -> [B*N*T, C] laid out as prep_features lays it out. A row outside [0, V)
+    reads nothing, gives zero output rows and sets err ([1] int32, sticky)."""
+    _check_cuda(store, rows, err)
+    assert store.dtype in (F32, BF16) and store.is_contiguous() and store.dim() in (3, 4)
+    assert (store.shape[2] if store.dim() == 4 else 1) == T, (tuple(store.shape), T)
+    assert rows.dtype == torch.int32 and rows.dim() == 1 and rows.is_contiguous()
+    assert err is not None and err.dtype == torch.int32 and err.numel() >= 1
+    V, N, C = store.shape[0], store.shape[1], store.shape[-1]
+    B = rows.numel()
+    out = _empty((B * N * T, C), out_dtype, store)
+    _lib.check(_v("prep_features_gather", out_dtype)(_ptr(store), 1 if store.dtype == BF16 else 0, V, N, _ptr(rows), B,
+                                                     _ptr(out), T, C, 1 if do_tanh else 0, 1 if time_major else 0, float(p),
+                                                     int(seed), int(stream_id), _ptr(err), _stream()),
+               "dvgr_prep_features_gather")
+    return out
+
+
 def dropout_raw(x, p, seed, stream_id, out=None):
     assert x.is_contiguous()
     if out is None:

@@ -357,6 +357,14 @@ int dvgr_prep_features(const float* in, void* out, long long S, int T, int C, in
  * features of the reference's DataLoader (DataLoader.py:61-84) put on the host link (SURVEY.md §8f.3). */
 int dvgr_prep_features_ex(const void* in, int in_is_bf16, void* out, long long S, int T, int C, int do_tanh,
                           int time_major, float p, unsigned long long seed, unsigned int drop_stream, void* stream);
+/* The same pass over a batch gathered from a device-resident feature store: store [V][N][T][C] (fp32, or bf16 when
+ * store_is_bf16), rows [B] int32 device -> out exactly as dvgr_prep_features_ex(store[rows], S = B*N, ...) writes it (same
+ * layout, same dropout mask). Replaces the per-sample HDF5 reads of DataLoader.py:61-84 and the host-to-device copy of the
+ * batch in front of Preprocessing.py:220-223 (appearance: T = 16, time_major, do_tanh) and models.py:74 (motion: T = 1).
+ * A row outside [0, V) is not read: its output rows are zero and *err (device int32, sticky: never cleared here) is set to 1. */
+int dvgr_prep_features_gather(const void* store, int store_is_bf16, long long V, int N, const int* rows, int B, void* out,
+                              int T, int C, int do_tanh, int time_major, float p, unsigned long long seed,
+                              unsigned int drop_stream, int* err, void* stream);
 int dvgr_cast_rows(const float* in, long long ld_in, void* out, long long ld_out, int rows, int cols, int out_cols,
                    int lstm_H, void* stream);
 /* n (<= 8) dvgr_cast_rows problems sharing ld_out / out_cols / lstm_H in one launch: the bf16 (gate-interleaved) copies of
@@ -486,6 +494,9 @@ int dvgr_bn_bwd_ex_f32(const void* dy, const void* x, int x_is_f32, int B, int D
                    int stats_only, void* stream);
 int dvgr_prep_features_ex_f32(const void* in, int in_is_bf16, void* out, long long S, int T, int C, int do_tanh,
                           int time_major, float p, unsigned long long seed, unsigned int drop_stream, void* stream);
+int dvgr_prep_features_gather_f32(const void* store, int store_is_bf16, long long V, int N, const int* rows, int B, void* out,
+                                  int T, int C, int do_tanh, int time_major, float p, unsigned long long seed,
+                                  unsigned int drop_stream, int* err, void* stream);
 int dvgr_dropout_f32(const void* in, void* out, long long n, float p, unsigned long long seed, unsigned int drop_stream,
                  void* stream);
 int dvgr_act_bwd_f32(const void* dy, const void* y, void* out, long long n, int act, int accumulate, float p,
